@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- decode tokens/s of a synthetic Llama-3-8B "v8-k65536-256" VPTQ stack on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One step = one decode token (batch 1) through every VPTQ-quantized linear of Llama-3-8B:
 32 layers x (q 4096x4096, k/v 1024x4096, o 4096x4096, gate/up 14336x4096, down 4096x14336),
@@ -424,12 +424,24 @@ def make_step(m, stack, device, dtype, rank, world, flags, tp_mode="nccl"):
         return x
 
     step.tp_error = tp_error if p2p else None
+    step.last_layer = buf      # after a step: the last decoder layer's projections (q, k, v, o, gate, up)
     return x_in, step, launches
 
 
 def _log(msg):
     if os.environ.get("BENCH_VERBOSE"):
         print(f"[bench r{os.environ.get('RANK', '0')} {time.strftime('%H:%M:%S')}] {msg}", file=sys.stderr, flush=True)
+
+
+def dump_outputs(out_dir, hidden, last_layer):
+    """What the last timed step computed, as float32 .npy files: the hidden state the step returns and, on one GPU,
+    the last layer's projections (k, v and up feed nothing downstream, so the hidden state alone would not show them).
+    The weights and the token are seeded, so two builds can be compared file for file."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"hidden": hidden, **{f"last_layer_{n}": t for n, t in last_layer.items()}}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def run_ours(args):
@@ -539,6 +551,8 @@ def run_ours(args):
             tp_err = int(te.item())
         assert tp_err == 0, "a tensor-parallel flag wait timed out"
         h_final = h_out.clone()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, h_out, step.last_layer if world == 1 else {})
 
         # ---- `e2e`: host buffers, H2D + D2H inside the timed region, per-step sync ------------------
         e2e_steps = args.steps
@@ -887,7 +901,13 @@ def main():
     ap.add_argument("--debug-layers", type=int, default=0, help="debugging only: truncate the model (invalid as a result)")
     ap.add_argument("--model", default="llama3-8b", choices=sorted(MODELS))
     ap.add_argument("--no-check", action="store_true", help="skip the unsharded recomputation of the token")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last timed step to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

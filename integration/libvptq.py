@@ -2,8 +2,8 @@
 directory's parent on sys.path as package `vptq`) and the reference's own python -- `vptq/ops/quant_gemm.py:22-26`
 does `import vptq.libvptq as vptq_ops` -- runs on libvptq_b200.so through the C ABI of include/vptq_b200.h.
 The three functions below have the signatures of the reference's pybind11 module (csrc/ops.cc:9-38,44-55).
-tests/test_host_logic.py::test_reference_python_binds_our_library_through_the_stub loads the reference's
-quant_gemm.py with this module in place."""
+tests/test_host_logic.py::test_reference_python_binds_our_library_through_the_stub replays against this module
+the calls the reference's quant_gemm.py makes into it (recorded by oracle/make_stub_calls.py)."""
 import ctypes, torch
 from vptq_b200 import native          # LinearDesc (= struct vptq_linear_desc), lib(), check(), workspace()
 
